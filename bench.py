@@ -18,6 +18,9 @@ independent synthetic streams (noise*0.1 + sine sweep).  A "step" is `passes_per
   cpu_baseline: the CPU oracle port timed on this box's host cores on a bounded sample
 
 `--impl reference` times the reference's CPU implementation of the same path (oracle port / compiled reference).
+`--dump-outputs DIR` writes DIR/pixels_argb.npy after the timed steps: the pixel columns of the last step for a fixed, seeded
+sample of (stream, column) pairs, as float32 [column][row][A, R, G, B].  The inputs are seeded too, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -43,6 +46,8 @@ STREAM_SECONDS = 20.0
 STREAMS_PER_GPU = 256
 WORKLOAD = dict(workload="cfg2-batch", sample_rate=48000, fft_size=N_FFT, hop=HOP, channels=CHANNELS, window="hann",
                 mix="absmean", palette="jade256", range_db=[-50, 50], rows=ROWS, pixel="ARGB32")
+DUMP_COLUMNS = 3072  # at most: 3072 x 1025 rows x 4 channels x 4 B = 50 MB for the cfg2-batch workload
+DUMP_BYTES = 64_000_000  # cap for any --geometry: the whole output (1.97 GB per GPU for cfg2-batch) is too large to keep
 
 
 def workload_config(world):
@@ -160,6 +165,21 @@ def cpu_baseline(sample_seconds=12.0, threads=None):
                 sample=f"{nstreams} streams x 2.0 s of the cfg2-batch workload ({frames} frames); {what}; "
                        f"1-thread rate {fps1:.0f} frames/s (calibration {cal:.1f} s)",
                 single_thread_value=fps1)
+
+
+def dump_outputs(out_dir, d_pix):
+    """DIR/pixels_argb.npy: the columns of d_pix [streams][columns][rows] (ARGB32 words) at a seeded sample of (stream, column)
+    pairs, split into their A, R, G, B bytes as float32 (exact)."""
+    import numpy as np
+    import torch
+    flat = d_pix.reshape(-1, d_pix.shape[-1])
+    ncols = min(flat.shape[0], DUMP_COLUMNS, DUMP_BYTES // (flat.shape[1] * 4 * 4))
+    idx = np.sort(np.random.default_rng(20240601).choice(flat.shape[0], ncols, replace=False))
+    sel = flat[torch.from_numpy(idx).to(flat.device)]
+    argb = torch.stack([(sel >> shift) & 0xFF for shift in (24, 16, 8, 0)], dim=-1).to(torch.float32)
+    out = pathlib.Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "pixels_argb.npy", argb.cpu().numpy())
 
 
 def run_reference(args):
@@ -292,6 +312,8 @@ def run_ours(args):
     max_ms = sharding.reduce_max(total_ms, dev)  # the slowest rank defines the job time
     value = frames_step * steps * world / (max_ms * 1e-3)
     kernel_ms = statistics.mean(per_launch_ms) / passes  # one pass = the main kernel + the launch for the boundary columns
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_pix)  # d_pix still holds the last timed pass: later legs use other buffers
 
     # ---- 1-GPU == N-GPU evidence on separate devices: rank 0 renders stream 0 of every other rank (same seed, same engine
     # configuration) and compares a checksum of the pixel columns with the one that rank computed itself
@@ -455,7 +477,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--only-kernel", action="store_true", help="device-resident loop only (for ncu)")
     ap.add_argument("--geometry", default=None, help="experiments only: FFT,HOP,CHANNELS instead of the cfg2-batch workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's pixel columns to DIR/pixels_argb.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference's CPU bench entry point returns no outputs")
     if args.geometry:
         global N_FFT, HOP, CHANNELS, ROWS, BYTES_ALG, WORKLOAD
         N_FFT, HOP, CHANNELS = (int(v) for v in args.geometry.split(","))

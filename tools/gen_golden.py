@@ -14,8 +14,11 @@
 
   paint_ref.npz    -- what the REFERENCE's own SpectrogramComponent::paint draws (crop rectangle of the spectrogram blit, the
                       tick values / label boxes of both axes, the colourbar pixels) for a few sizes and slider positions.
+  oracle_vs_reference.npz -- the reference's side of every comparison in tests/test_oracle_vs_reference.py (sha256 per value;
+                      the committed file holds the oracle's side, see that test's docstring).
 
     python tools/gen_golden.py          (everything)      python tools/gen_golden.py paint   (paint_ref.npz only)
+    python tools/gen_golden.py oracle_vs_reference        (oracle_vs_reference.npz only)
 """
 import hashlib
 import pathlib
@@ -188,7 +191,20 @@ def paint_reference():
     print("paint_ref.npz", len(out), "arrays")
 
 
+def oracle_vs_reference():
+    """tests/golden/oracle_vs_reference.npz: what the compiled reference returns in each scenario of
+    tests/test_oracle_vs_reference.py (a sha256 per value)."""
+    assert O.have_ref_spec(), "oracle/_ref/libjade_ref.so lacks the Spectrogram glue: run `make -C oracle` where the reference exists"
+    import test_oracle_vs_reference as T
+    out = {key: np.stack([T.digest(v) for _, v in run(True)]) for key, run in T.scenarios().items()}
+    np.savez_compressed(OUT / "oracle_vs_reference.npz", **out)
+    print("oracle_vs_reference.npz", len(out), "arrays")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "oracle_vs_reference":
+        oracle_vs_reference()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "paint":
         paint_reference()
         sys.exit(0)
@@ -197,3 +213,4 @@ if __name__ == "__main__":
     pipeline()
     reference_class()
     paint_reference()
+    oracle_vs_reference()
