@@ -595,7 +595,7 @@ int launch_one(jade_engine* e, const KernelChoice& kc, KParams& P, cudaStream_t 
             return fail(e, JADE_ERR_STATE, "scratch not sized for grid %d", grid);
     }
     void* args[] = {(void*)&P};
-    static const bool trace = getenv("JADE_TRACE_LAUNCH") != nullptr; // experiments: one line per launch on stderr
+    static const bool trace = getenv("JADE_TRACE_LAUNCH") != nullptr; // one line per launch on stderr (tests/test_gpu_routes64.py)
     kernel_fn fn = (P.db && kc.fn_db) ? kc.fn_db : kc.fn;
     // long runs of evenly spaced columns, a quarter frame apart: the instantiation that walks contiguous columns per warp
     static const bool no_run = [] { const char* v = getenv("JADE_PK_LOAD"); return v && !strcmp(v, "norun"); }(); // experiments
@@ -605,9 +605,14 @@ int launch_one(jade_engine* e, const KernelChoice& kc, KParams& P, cudaStream_t 
         fn = P.db ? kc.fn_run_db : ((P.pal_u8 && kc.fn_run_u8) ? kc.fn_run_u8 : kc.fn_run);
     else if (!P.db && P.pal_u8 && kc.fn_u8 && fn == kc.fn)
         fn = kc.fn_u8;
-    if (trace)
-        fprintf(stderr, "[jade] %s%s grid %d x %d threads, smem %d, blocks/SM %d, frames %lld\n", kc.name, (fn == kc.fn_run || fn == kc.fn_run_db || fn == kc.fn_run_u8) ? "+run" : "", grid,
-                kc.threads, kc.smem, kc.blocks_per_sm, frames);
+    if (trace) {
+        // the suffixes name the instantiation: +run (long-run ring), +db (dB-storing form), +u8 (saturating u8 palette form)
+        const bool is_run = fn == kc.fn_run || fn == kc.fn_run_db || fn == kc.fn_run_u8;
+        const bool is_db = fn == kc.fn_db || fn == kc.fn_run_db;
+        const bool is_u8 = fn == kc.fn_u8 || fn == kc.fn_run_u8;
+        fprintf(stderr, "[jade] %s%s%s%s grid %d x %d threads, smem %d, blocks/SM %d, frames %lld\n", kc.name, is_run ? "+run" : "",
+                is_db ? "+db" : "", is_u8 ? "+u8" : "", grid, kc.threads, kc.smem, kc.blocks_per_sm, frames);
+    }
     if (P.ring_w > 0) {
         // streaming push: programmatic dependent launch behind ingest_kernel (every STFT kernel calls grid_dep_wait()
         // after its table prologue, jade_kernels.cuh)
