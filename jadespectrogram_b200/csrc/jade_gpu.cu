@@ -373,18 +373,21 @@ int choose_kernel(jade_engine* e)
         e->kc_edge = ke;
     } else if (N <= 2048) {
         const int T = N / 64;
+        // N >= 128 without the general epilogue only lands here when the palette does not fit the packed kernel: the warp
+        // kernel of these sizes exists with the general epilogue only (jade_k_warp_*.cu)
+        const bool gen = po || T > 1;
         kc.family = 0;
         kc.threads = jade::WARP_KERNEL_WARPS * 32;
         kc.units_per_block = jade::WARP_KERNEL_WARPS * (32 / T);
         snprintf(kc.name, sizeof kc.name, "warp<%d>", T);
-        kc.fn = jade_k::warp_kernel(T, mu, po);
+        kc.fn = jade_k::warp_kernel(T, mu, gen);
         switch (T) {
-        case 1: kc.smem = jade::WarpCfg<1>::smem_bytes(e->npal, po); break;
-        case 2: kc.smem = jade::WarpCfg<2>::smem_bytes(e->npal, po); break;
-        case 4: kc.smem = jade::WarpCfg<4>::smem_bytes(e->npal, po); break;
-        case 8: kc.smem = jade::WarpCfg<8>::smem_bytes(e->npal, po); break;
-        case 16: kc.smem = jade::WarpCfg<16>::smem_bytes(e->npal, po); break;
-        case 32: kc.smem = jade::WarpCfg<32>::smem_bytes(e->npal, po); break;
+        case 1: kc.smem = jade::WarpCfg<1>::smem_bytes(e->npal, gen); break;
+        case 2: kc.smem = jade::WarpCfg<2>::smem_bytes(e->npal, gen); break;
+        case 4: kc.smem = jade::WarpCfg<4>::smem_bytes(e->npal, gen); break;
+        case 8: kc.smem = jade::WarpCfg<8>::smem_bytes(e->npal, gen); break;
+        case 16: kc.smem = jade::WarpCfg<16>::smem_bytes(e->npal, gen); break;
+        case 32: kc.smem = jade::WarpCfg<32>::smem_bytes(e->npal, gen); break;
         default: return fail(e, JADE_ERR_ARG, "unsupported fft_size %d", N);
         }
         if (!kc.fn) return fail(e, JADE_ERR_ARG, "unsupported fft_size %d", N);
@@ -437,7 +440,6 @@ int choose_kernel(jade_engine* e)
         default: return fail(e, JADE_ERR_ARG, "unsupported fft_size %d", N);
         }
         if (!kc.fn) return fail(e, JADE_ERR_ARG, "unsupported fft_size %d", N);
-        if (kc.fn_db) CU(e, cudaFuncSetAttribute((const void*)kc.fn_db, cudaFuncAttributeMaxDynamicSharedMemorySize, kc.smem));
     } else if (N == 65536) {
         static const bool one_cta = [] { const char* v = getenv("JADE_N65536"); return v && !strcmp(v, "cta2"); }(); // experiments
         kc.threads = 32 * 16;
@@ -468,6 +470,7 @@ int choose_kernel(jade_engine* e)
         return fail(e, JADE_ERR_ARG, "kernel %s needs %d bytes of shared memory with a %d-colour palette (limit %d)", kc.name, kc.smem,
                     e->npal, e->smem_optin);
     CU(e, cudaFuncSetAttribute((const void*)kc.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, kc.smem));
+    if (kc.fn_db) CU(e, cudaFuncSetAttribute((const void*)kc.fn_db, cudaFuncAttributeMaxDynamicSharedMemorySize, kc.smem));
     int occ = 0;
     CU(e, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, (const void*)kc.fn, kc.threads, kc.smem));
     if (occ < 1) return fail(e, JADE_ERR_CUDA, "kernel %s does not fit on an SM (smem %d)", kc.name, kc.smem);
@@ -610,8 +613,9 @@ int launch_one(jade_engine* e, const KernelChoice& kc, KParams& P, cudaStream_t 
         const bool is_run = fn == kc.fn_run || fn == kc.fn_run_db || fn == kc.fn_run_u8;
         const bool is_db = fn == kc.fn_db || fn == kc.fn_run_db;
         const bool is_u8 = fn == kc.fn_u8 || fn == kc.fn_run_u8;
-        fprintf(stderr, "[jade] %s%s%s%s grid %d x %d threads, smem %d, blocks/SM %d, frames %lld\n", kc.name, is_run ? "+run" : "",
-                is_db ? "+db" : "", is_u8 ? "+u8" : "", grid, kc.threads, kc.smem, kc.blocks_per_sm, frames);
+        fprintf(stderr, "[jade] %s%s%s%s grid %d x %d threads, smem %d, blocks/SM %d, frames %lld, units/block %d\n", kc.name,
+                is_run ? "+run" : "", is_db ? "+db" : "", is_u8 ? "+u8" : "", grid, kc.threads, kc.smem, kc.blocks_per_sm, frames,
+                kc.units_per_block);
     }
     if (P.ring_w > 0) {
         // streaming push: programmatic dependent launch behind ingest_kernel (every STFT kernel calls grid_dep_wait()
